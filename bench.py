@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: audio samples/s denoised (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload at N=1 = BASELINE.json configs[1]: 64 ch x 10 min synthetic 48 kHz, stationary reduce_noise,
 n_fft=1024 hop=256 (1.8432 G samples per step).  A step is one full pass of the hot path
@@ -18,10 +18,12 @@ n_fft=1024 hop=256 (1.8432 G samples per step).  A step is one full pass of the 
   configs_extra  BASELINE configs 3 (non-stationary, n_fft 2048) and 4 (TorchGate 256 x 10 s @ 16 kHz): device-resident
                samples/s, whole-step roofline fraction, CPU legs
   cpu_baseline the reference's CPU path with n_jobs=-1 on this box's host cores on a bounded sample of the workload
-               (the unmodified reference when /root/reference is importable, else oracle/ref_port.py -- the same
-               scipy.signal calls and joblib fan-out), plus n_jobs=1
+               (oracle/ref_port.py: the reference's scipy.signal calls and joblib fan-out), plus n_jobs=1
 
 --impl reference times that CPU path alone (rank 0 only under torchrun).
+--dump-outputs DIR writes the waveform the last timed step computed to DIR/denoised.npy (float32; every row at a fixed,
+seeded sample of column blocks when the whole output exceeds 64 MB), so that two builds can be compared on the same
+seeded input.
 """
 import argparse
 import json
@@ -41,7 +43,8 @@ N_SAMPLES = 28_800_000            # 10 min @ 48 kHz
 METRIC = "audio samples/sec denoised"
 UNIT = "samples/s"
 ALGO_BYTES_PER_SAMPLE = 8          # float32 in + float32 out (SURVEY.md section 8d)
-REFERENCE_DIR = "/root/reference"
+DUMP_BYTES = 60_000_000            # --dump-outputs: array bytes written, under 64 MB with the .npy header
+DUMP_BLOCK = 4096
 
 
 def measured_hbm_peak():
@@ -154,17 +157,17 @@ def synth_host(np, C, n):
     return y
 
 
-def _reference_module():
-    """The unmodified reference, when its checkout is present (the build container; not the GPU box)."""
-    if not os.path.isdir(os.path.join(REFERENCE_DIR, "noisereduce")):
-        return None
-    try:
-        if REFERENCE_DIR not in sys.path:
-            sys.path.append(REFERENCE_DIR)
-        import noisereduce as nr      # noqa: F401
-        return nr
-    except Exception:
-        return None
+def dump_outputs(np, torch, directory, name, y):
+    """Writes the [rows, n] float32 tensor `y` as directory/name.npy: whole when it fits in DUMP_BYTES, else every row
+    at a fixed set of DUMP_BLOCK-sample column blocks (seeded, sorted; the same for the same shape)."""
+    rows, n = y.shape
+    if rows * n * 4 > DUMP_BYTES:
+        blocks = DUMP_BYTES // (rows * DUMP_BLOCK * 4)
+        starts = np.sort(np.random.default_rng(0).choice(n // DUMP_BLOCK, size=blocks, replace=False)) * DUMP_BLOCK
+        cols = torch.from_numpy((starts[:, None] + np.arange(DUMP_BLOCK)).reshape(-1)).to(y.device)
+        y = y.index_select(1, cols)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, f"{name}.npy"), y.to(torch.float32).cpu().numpy())
 
 
 def cpu_reference_run(steps, warmup, channels=16, minutes=10.0, stationary=True, n_fft=1024, with_single_job=True):
@@ -175,24 +178,18 @@ def cpu_reference_run(steps, warmup, channels=16, minutes=10.0, stationary=True,
     import numpy as np
     import scipy
     import joblib
+    from oracle import ref_port
+    from oracle import spectral_gate_oracle as O
     cores = os.cpu_count() or 1
     n = int(minutes * 60 * SR)
     y = synth_host(np, channels, n)
-    nr = _reference_module()
-    kind = "reference" if nr is not None else "port"
     kw = dict(stationary=stationary, n_fft=n_fft)
     if n_fft == 1024:
         kw["hop_length"] = 256
-    if nr is not None:
-        def run(arr, jobs):
-            return nr.reduce_noise(y=arr, sr=SR, n_jobs=jobs, **kw)
-    else:
-        from oracle import ref_port
-        from oracle import spectral_gate_oracle as O
-        cfg = O.GateConfig(sr=SR, **kw)
+    cfg = O.GateConfig(sr=SR, **kw)
 
-        def run(arr, jobs):
-            return ref_port.reduce_noise(arr, SR, cfg, n_jobs=jobs)
+    def run(arr, jobs):
+        return ref_port.reduce_noise(arr, SR, cfg, n_jobs=jobs)
     for _ in range(max(0, min(warmup, 1))):           # one warm-up spawns the loky pool (BASELINE.md section 3)
         run(y[:, : 2 * 600000 + 1], -1)
     times = []
@@ -202,10 +199,10 @@ def cpu_reference_run(steps, warmup, channels=16, minutes=10.0, stationary=True,
         times.append(time.perf_counter() - t0)
     dt = sum(times) / len(times)
     n_chunks = (n - 1) // 600000 + 1
-    res = dict(value=channels * n / dt, unit=UNIT, cores=cores, kind=kind, n_jobs=-1, host_cores=cores,
+    res = dict(value=channels * n / dt, unit=UNIT, cores=cores, kind="port", n_jobs=-1, host_cores=cores,
                busy_workers_max=min(cores, n_chunks), seconds_per_step=dt,
                sample=f"{channels} of 64 ch x all {n_chunks} chunks of 600000 samples ({channels * n / 1e6:.0f} Msamples) per step, "
-                      f"{'noisereduce.reduce_noise' if kind == 'reference' else 'oracle/ref_port.py (same scipy.signal calls)'}"
+                      "oracle/ref_port.py (same scipy.signal calls)"
                       f"(n_jobs=-1): joblib over chunks, channels serial inside a chunk job -> samples/s independent of the channel count",
                versions={"numpy": np.__version__, "scipy": scipy.__version__, "joblib": joblib.__version__})
     if with_single_job:
@@ -217,31 +214,17 @@ def cpu_reference_run(steps, warmup, channels=16, minutes=10.0, stationary=True,
 
 
 def torchgate_cpu_leg(rows=16):
-    """Config 4 CPU leg: the reference's TorchGate on CPU when importable, else torch ops restating it (oracle)."""
+    """Config 4 CPU leg: the reference's TorchGate restated in numpy (oracle), single thread."""
     import numpy as np
     import torch
-    threads = torch.get_num_threads()
     g = torch.Generator().manual_seed(1234)
     x = 0.05 * torch.randn((rows, 160000), generator=g)
-    nr = _reference_module()
     try:
-        if nr is not None:
-            from noisereduce.torchgate import TorchGate as RefGate
-            tg = RefGate(sr=16000)
-            with torch.no_grad():
-                tg(x[:2])
-                t0 = time.perf_counter()
-                tg(x)
-                dt = time.perf_counter() - t0
-            kind = "reference"
-        else:
-            from oracle import torchgate_oracle as TO
-            t0 = time.perf_counter()
-            TO.torchgate_forward(x.numpy().astype(np.float64), sr=16000)
-            dt = time.perf_counter() - t0
-            kind = "port (numpy restatement, single thread)"
-            threads = 1
-        return {"value": rows * 160000 / dt, "unit": UNIT, "kind": kind, "threads": threads,
+        from oracle import torchgate_oracle as TO
+        t0 = time.perf_counter()
+        TO.torchgate_forward(x.numpy().astype(np.float64), sr=16000)
+        dt = time.perf_counter() - t0
+        return {"value": rows * 160000 / dt, "unit": UNIT, "kind": "port (numpy restatement, single thread)", "threads": 1,
                 "sample": f"{rows} of 256 rows x 160000 samples"}
     except Exception as exc:
         return {"value": None, "error": repr(exc)[:160]}
@@ -337,7 +320,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip parity / configs_extra / e2e_numpy (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output to DIR/denoised.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -353,7 +339,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = min(args.steps, 3)
+        steps = args.steps
         r = cpu_reference_run(steps, args.warmup, channels=32, minutes=args.minutes)
         cb = {k: r[k] for k in ("value", "unit", "cores", "kind", "sample", "n_jobs", "host_cores", "busy_workers_max",
                                 "versions", "n_jobs_1_value") if k in r}
@@ -496,6 +482,8 @@ def main():
         dist.all_reduce(okf, op=dist.ReduceOp.MIN)
         gather_verified = bool(okf.item() > 0)
     ref_out = out if out is not None else (ps.buf[rank] if ps is not None else pg.buf[rank])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(np, torch, args.dump_outputs, "denoised", ref_out if world == 1 else full.reshape(world * C, n))
 
     # ---- end to end through the C ABI with host buffers ----------------------------------------------
     e2e = None

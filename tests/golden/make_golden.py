@@ -28,6 +28,7 @@ import noisereduce as nr  # noqa: E402  (the reference)
 from noisereduce.spectralgate.stationary import SpectralGateStationary  # noqa: E402
 from noisereduce.torchgate import TorchGate  # noqa: E402
 
+from tests.golden.fixtures import save  # noqa: E402
 from tests.synth_host import synth_small, synth_torchgate  # noqa: E402
 
 VERSIONS = np.array(
@@ -60,8 +61,8 @@ def main():
     # ---- config 1: assets/fish.wav (int16 mono 44.1 kHz), defaults -------------------------
     rate, fish = wavfile.read(os.path.join(REF, "assets", "fish.wav"))
     fish_f32 = (fish / 32768).astype(np.float32)
-    np.savez_compressed(
-        os.path.join(HERE, "fish_cfg1.npz"),
+    save(
+        "fish_cfg1",
         versions=VERSIONS, sr=rate, y=fish,
         out_stationary=nr.reduce_noise(y=fish, sr=rate, stationary=True),
         out_nonstationary=nr.reduce_noise(y=fish, sr=rate, stationary=False),
@@ -75,8 +76,8 @@ def main():
     y = synth_small()                       # float32 [2, 30000]
     kw = dict(chunk_size=12000, padding=1500)
     yn = y[:, 3000:11000]
-    np.savez_compressed(
-        os.path.join(HERE, "synth_small.npz"),
+    save(
+        "synth_small",
         versions=VERSIONS, sr=sr, y=y,
         out_stat_chunked=nr.reduce_noise(y=y, sr=sr, stationary=True, **kw),
         thresh_stat_chunked=stationary_thresh(y, sr, **kw),
@@ -92,8 +93,8 @@ def main():
     )
 
     # ---- get_traces sub-ranges: chunk-grid branch and the single-padded-chunk branch ----------
-    np.savez_compressed(
-        os.path.join(HERE, "synth_traces.npz"),
+    save(
+        "synth_traces",
         versions=VERSIONS, sr=sr,
         chunks_13000_28000=traces(y, sr, 13000, 28000, **kw),          # chunks 1..2 of 3, trimmed
         chunks_500_24500=traces(y, sr, 500, 24500, **kw),              # chunks 0..2, end on a chunk edge + 500
@@ -103,8 +104,8 @@ def main():
 
     # ---- STFT geometries off the default (general-geometry kernel family) ------------------------
     yi16 = np.round(y * 20000).astype(np.int16)
-    np.savez_compressed(
-        os.path.join(HERE, "synth_geometry.npz"),
+    save(
+        "synth_geometry",
         versions=VERSIONS, sr=sr,
         stat_512=nr.reduce_noise(y=y, sr=sr, stationary=True, n_fft=512, **kw),
         thresh_512=stationary_thresh(y, sr, n_fft=512, **kw),
@@ -130,8 +131,8 @@ def main():
     tg_n = TorchGate(sr=sr, nonstationary=True)
     tg_x = TorchGate(sr=sr, prop_decrease=0.7)
     xn = xt64[:1, :6000]
-    np.savez_compressed(
-        os.path.join(HERE, "torchgate_small.npz"),
+    save(
+        "torchgate_small",
         versions=VERSIONS, sr=sr, x=x,
         window=torch.hann_window(1024).numpy(),
         filt=tg_s.smoothing_filter.numpy()[0, 0],
@@ -144,8 +145,8 @@ def main():
     # ---- TorchGate off the default STFT geometry (general family, torch surface) -------------------
     xg = x[:2, :12000]
     xg64 = torch.from_numpy(xg).double()
-    np.savez_compressed(
-        os.path.join(HERE, "torchgate_geometry.npz"),
+    save(
+        "torchgate_geometry",
         versions=VERSIONS, sr=sr,
         window_400=torch.hann_window(400).numpy(),
         stat_512_400_100_f64=TorchGate(sr=sr, n_fft=512, win_length=400, hop_length=100)(xg64).numpy(),

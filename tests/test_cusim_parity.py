@@ -11,6 +11,7 @@ from noisereduce_b200 import _cabi
 from oracle import spectral_gate_oracle as O
 from tests import parity_cases as P
 from tests.cusim_util import cusim_library
+from tests.golden import fixtures as golden
 from tests.synth_host import synth_small
 
 SR = 16000
@@ -581,10 +582,9 @@ def test_prop_decrease_outside_unit_interval_like_the_reference(lib):
 
 def test_reference_test_suite_scenarios_on_simulator(lib, monkeypatch, golden_dir):
     """test_reduction.py:6-56 of the reference (its four numpy-path scenarios) on the first 50000 samples of its asset."""
-    import os
     monkeypatch.setattr(_cabi, "_LIB", lib)
     import noisereduce_b200 as nr
-    f = np.load(os.path.join(golden_dir, "fish_cfg1.npz"))
+    f = golden.load(golden_dir, "fish_cfg1")
     sr = int(f["sr"])
     for name, y, kw in P.reference_test_suite_scenarios(f["y"], sr, n=50000):
         if name == "stationary_without_noise_clip":

@@ -1,12 +1,11 @@
 """Parity on a real B200 (-m gpu), through the C ABI of the nvcc-built libb200gate.so."""
-import os
-
 import numpy as np
 import pytest
 
 from noisereduce_b200 import _cabi
 from oracle import spectral_gate_oracle as O
 from tests import parity_cases as P
+from tests.golden import fixtures as golden
 from tests.synth_host import synth_small
 
 pytestmark = pytest.mark.gpu
@@ -91,10 +90,10 @@ def test_nonstationary(lib, golden_dir):
     res = P.check_nonstationary(lib, yy, cfg, tap_unit=(1, 1))
     assert res["mask_err"] < P.MASK_TOL_NONSTAT and res["out_relinf"] < P.OUT_TOL_TIGHT * 5, res
     # golden: reference outputs
-    s = np.load(os.path.join(golden_dir, "synth_small.npz"))
+    s = golden.load(golden_dir, "synth_small")
     out = nr.reduce_noise(y=s["y"], sr=int(s["sr"]), stationary=False, chunk_size=12000, padding=1500)
     assert P.relinf(out, s["out_nonstat_chunked"]) < P.OUT_TOL
-    f = np.load(os.path.join(golden_dir, "fish_cfg1.npz"))
+    f = golden.load(golden_dir, "fish_cfg1")
     out = nr.reduce_noise(y=f["y"], sr=int(f["sr"]), stationary=False)
     assert np.abs(out.astype(np.int32) - f["out_nonstationary"].astype(np.int32)).max() <= 1
 
@@ -113,7 +112,7 @@ def test_nonstationary_n_fft_2048_config3(lib, golden_dir):
         assert res["T"] == 1290
         assert res["spec_err"] < P.SPEC_TOL and res["mask_err"] < P.MASK_TOL_NONSTAT, res
         assert res["out_relinf"] < P.OUT_TOL_TIGHT * 5, res
-    s = np.load(os.path.join(golden_dir, "synth_small.npz"))
+    s = golden.load(golden_dir, "synth_small")
     out = nr.reduce_noise(y=s["y"].astype(np.float64), sr=int(s["sr"]), stationary=False, n_fft=2048,
                           time_constant_s=0.5, prop_decrease=0.9)
     assert out.dtype == np.float64 and P.relinf(out, s["out_nonstat_2048_f64"]) < P.OUT_TOL
@@ -155,14 +154,14 @@ def test_pooled_result_buffers(lib):
 
 def test_golden_fish_and_small(lib, golden_dir):
     import noisereduce_b200 as nr
-    f = np.load(os.path.join(golden_dir, "fish_cfg1.npz"))
+    f = golden.load(golden_dir, "fish_cfg1")
     out = nr.reduce_noise(y=f["y"], sr=int(f["sr"]), stationary=True)
     assert out.dtype == np.int16 and out.shape == f["y"].shape
     assert np.abs(out.astype(np.int32) - f["out_stationary"].astype(np.int32)).max() <= 1      # <= 1 LSB
     yf = (f["y"] / 32768).astype(np.float32)
     out = nr.reduce_noise(y=yf, sr=int(f["sr"]), stationary=True)
     assert P.relinf(out, f["out_stationary_f32"]) < P.OUT_TOL
-    s = np.load(os.path.join(golden_dir, "synth_small.npz"))
+    s = golden.load(golden_dir, "synth_small")
     kw = dict(chunk_size=12000, padding=1500)
     y, sr = s["y"], int(s["sr"])
     assert P.relinf(nr.reduce_noise(y=y, sr=sr, stationary=True, **kw), s["out_stat_chunked"]) < P.OUT_TOL
@@ -177,7 +176,7 @@ def test_get_traces_subranges_golden(lib, golden_dir):
     """SpectralGate.get_traces(start_frame, end_frame) against reference outputs (base.py:167-226): only
     the selected units run, and the result equals the reference's chunk-grid / single-chunk branches."""
     from noisereduce_b200.spectralgate.stationary import SpectralGateStationary
-    g = np.load(os.path.join(golden_dir, "synth_traces.npz"))
+    g = golden.load(golden_dir, "synth_traces")
     y = synth_small()
     args = dict(y_noise=None, n_std_thresh_stationary=1.5, clip_noise_stationary=True, n_fft=1024, win_length=None,
                 hop_length=None, time_constant_s=2.0, freq_mask_smooth_hz=500, time_mask_smooth_ms=50,
@@ -245,7 +244,7 @@ def test_torchgate_surface(lib, golden_dir):
     import torch
     from noisereduce_b200.torchgate import TorchGate
     from oracle import torchgate_oracle as TO
-    g = np.load(os.path.join(golden_dir, "torchgate_small.npz"))
+    g = golden.load(golden_dir, "torchgate_small")
     x = torch.from_numpy(g["x"]).cuda()
     sr = int(g["sr"])
     tol = 2e-5          # FP32 path vs the reference's float32 / float64 runs (its own f32-vs-f64 gap is 2.5e-7)
@@ -304,7 +303,7 @@ def test_batching_slabs_and_config5_geometry(lib):
 def test_reference_test_suite_scenarios(lib, golden_dir):
     """test_reduction.py:6-56 of the reference, through reduce_noise() on the GPU, against the oracle."""
     import noisereduce_b200 as nr
-    f = np.load(os.path.join(golden_dir, "fish_cfg1.npz"))
+    f = golden.load(golden_dir, "fish_cfg1")
     sr = int(f["sr"])
     for name, y, kw in P.reference_test_suite_scenarios(f["y"], sr):
         out = nr.reduce_noise(y=y, sr=sr, **kw)
@@ -320,7 +319,7 @@ def test_general_geometry_family_golden_and_stages(lib, golden_dir):
     kernels cross-checked against the general family on the same input."""
     import noisereduce_b200 as nr
     from tests.test_oracle_golden import GEOMETRY_CASES, NON_POW2_KEYS, geometry_input
-    g = np.load(os.path.join(golden_dir, "synth_geometry.npz"))
+    g = golden.load(golden_dir, "synth_geometry")
     for key, (kw, dt) in GEOMETRY_CASES.items():
         if key in NON_POW2_KEYS:
             continue                                   # test_non_power_of_two_n_fft_golden
@@ -366,7 +365,7 @@ def test_torchgate_general_geometry_golden(lib, golden_dir):
     from noisereduce_b200.torchgate import TorchGate
     from tests.synth_host import synth_torchgate
     from tests.test_oracle_golden import NON_POW2_KEYS, TG_GEOMETRY_CASES
-    g = np.load(os.path.join(golden_dir, "torchgate_geometry.npz"))
+    g = golden.load(golden_dir, "torchgate_geometry")
     x = synth_torchgate()[:2, :12000]
     for key, (kw, xn_idx, dt) in TG_GEOMETRY_CASES.items():
         if key in NON_POW2_KEYS:
@@ -386,7 +385,7 @@ def test_non_power_of_two_n_fft_golden(lib, golden_dir):
     from noisereduce_b200.torchgate import TorchGate
     from tests.synth_host import synth_torchgate
     from tests.test_oracle_golden import GEOMETRY_CASES, NON_POW2_KEYS, TG_GEOMETRY_CASES, geometry_input
-    g = np.load(os.path.join(golden_dir, "synth_geometry.npz"))
+    g = golden.load(golden_dir, "synth_geometry")
     for key, (kw, dt) in GEOMETRY_CASES.items():
         if key in NON_POW2_KEYS:
             out = nr.reduce_noise(y=geometry_input(dt), sr=16000, chunk_size=12000, padding=1500, **kw)
@@ -400,7 +399,7 @@ def test_non_power_of_two_n_fft_golden(lib, golden_dir):
         cfg = O.GateConfig(sr=SR, stationary=False, chunk_size=12000, padding=1500, time_constant_s=0.3, time_mask_smooth_ms=ms, **geo)
         r = P.check_nonstationary(lib, y, cfg, tap_unit=(2, 0))
         assert r["spec_err"] < 2e-7 and r["mask_err"] < 2e-7 and r["out_relinf"] < 2e-7, (geo, r)
-    gt = np.load(os.path.join(golden_dir, "torchgate_geometry.npz"))
+    gt = golden.load(golden_dir, "torchgate_geometry")
     x = synth_torchgate()[:2, :12000]
     for key, (kw, xn_idx, dt) in TG_GEOMETRY_CASES.items():
         if key in NON_POW2_KEYS:

@@ -3,13 +3,12 @@
 CPU-only.  The bar: integer outputs bit-equal; float outputs within 1e-12 relative (the oracle
 restates the same float64 arithmetic; only summation order inside the 2-D smoothing differs).
 """
-import os
-
 import numpy as np
 import pytest
 
 from oracle import spectral_gate_oracle as O
 from oracle import torchgate_oracle as TO
+from tests.golden import fixtures as golden
 from tests.synth_host import synth_small, synth_torchgate
 
 
@@ -23,17 +22,17 @@ def relinf(a, b):
 
 @pytest.fixture(scope="module")
 def fish(golden_dir):
-    return np.load(os.path.join(golden_dir, "fish_cfg1.npz"))
+    return golden.load(golden_dir, "fish_cfg1")
 
 
 @pytest.fixture(scope="module")
 def small(golden_dir):
-    return np.load(os.path.join(golden_dir, "synth_small.npz"))
+    return golden.load(golden_dir, "synth_small")
 
 
 @pytest.fixture(scope="module")
 def tgs(golden_dir):
-    return np.load(os.path.join(golden_dir, "torchgate_small.npz"))
+    return golden.load(golden_dir, "torchgate_small")
 
 
 def test_dft_primitive_matches_definition():
@@ -204,7 +203,7 @@ def test_ref_port_matches_reference(small, fish):
 def test_get_traces_subranges_match_reference(golden_dir):
     """SpectralGate.get_traces(start_frame, end_frame) (base.py:167-226): chunk-grid branch, and the
     single padded chunk whose right padding is real signal (base.py:222)."""
-    g = np.load(os.path.join(golden_dir, "synth_traces.npz"))
+    g = golden.load(golden_dir, "synth_traces")
     y = synth_small()
     cfg = O.GateConfig(sr=16000, stationary=True, chunk_size=12000, padding=1500)
     for key, (a, b) in {"chunks_13000_28000": (13000, 28000), "chunks_500_24500": (500, 24500),
@@ -241,7 +240,7 @@ def geometry_input(dtype):
 def test_non_default_stft_geometries_match_reference(golden_dir):
     """n_fft / win_length / hop_length off the defaults (base.py:79-86): odd window, hop not dividing the
     window, zero-padded FFT -- the oracle restates scipy's framing for all of them."""
-    g = np.load(os.path.join(golden_dir, "synth_geometry.npz"))
+    g = golden.load(golden_dir, "synth_geometry")
     for key, (kw, dt) in GEOMETRY_CASES.items():
         y = geometry_input(dt)
         cfg = O.GateConfig(sr=16000, chunk_size=12000, padding=1500, **kw)
@@ -270,7 +269,7 @@ TG_GEOMETRY_CASES = {
 def test_torchgate_non_default_geometries_match_reference(golden_dir):
     """TorchGate with n_fft / win_length / hop_length off the defaults: window centre-padded to n_fft, pad n_fft/2
     (torch.stft center=True), output (L // hop) * hop (torchgate.py:223-262)."""
-    g = np.load(os.path.join(golden_dir, "torchgate_geometry.npz"))
+    g = golden.load(golden_dir, "torchgate_geometry")
     x = synth_torchgate()[:2, :12000]
     for key, (kw, xn_idx, dt) in TG_GEOMETRY_CASES.items():
         xn = None if xn_idx is None else x[xn_idx].astype(np.float64)
