@@ -64,15 +64,12 @@ typedef struct b200gate_params {
     int32_t debug_guard_scale;  /* tests only: multiplies the FP32 guard band (0 = 1x), forcing more
                                  * bins through the FP64 re-decision path                          */
     int32_t reserve_sms;        /* SMs the persistent grids leave free (for a concurrent NCCL collective) */
-    int32_t path_flags;         /* kept cross-check variants of the same arithmetic (default 0).  bit 1: do not cache
-                                 * spectra between analysis and synthesis (re-transform instead; saves 8 KB of workspace per
-                                 * frame pair); bit 2: run the float64 general-geometry family even for a tuned geometry;
-                                 * bit 3: k1 streams the next frame pair's float32 sample rows into shared memory with
-                                 * cp.async (measured: no gain); bit 4: one unit per warp in the n_fft 1024 FFT kernels
-                                 * instead of the dual (packed f32x2) forms; bit 5: tile-based float-mask smoothing;
-                                 * bit 6: the non-stationary follower stores its forward sweep instead of regenerating
-                                 * it; bit 7: tap-loop float-mask smoothing instead of the box-sum form.  (bit 0 selected
-                                 * a single-pass experiment that was removed; it is ignored)                          */
+    int32_t path_flags;         /* force a path that some input needs onto any input (default 0).  bit 2: run the
+                                 * float64 general-geometry family even for a tuned geometry; bit 4: one unit per warp in
+                                 * the n_fft 1024 FFT kernels instead of the dual (packed f32x2) forms; bit 5: tile-based
+                                 * float-mask smoothing; bit 6: the non-stationary follower stores its forward sweep
+                                 * instead of regenerating it; bit 7: tap-loop float-mask smoothing instead of the
+                                 * box-sum form.  Bits 0, 1 and 3 selected variants that were removed; they are ignored */
     int64_t chunk_size;         /* <= 0: never chunk (torch surface / chunk_size=None)           */
     int64_t padding;
     double sr;

@@ -2,7 +2,7 @@
 //
 // The planner turns the reference's chunk loop (noisereduce/spectralgate/base.py:167-226) into a
 // table of independent (chunk, channel) units, sizes the device workspace, and launches
-// k1_analyze -> k_rowfloor -> k_smooth -> k2_synthesize per batch of units on the caller's stream.
+// k1_analyze -> k_rowfloor -> k_smooth -> k2c_synthesize per batch of units on the caller's stream.
 #include "../../include/b200gate.h"
 #include "gate_kernels_2k.cuh"
 #include "gate_synth.cuh"
@@ -893,8 +893,6 @@ int b200gate_create(const b200gate_params* p, b200gate_handle** out) {
         for (int dt = 0; dt < 3; ++dt)
             B200_WITH_DTYPE(dt, {
                 cudaFuncSetAttribute(k1_analyze<8, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k1_smem_floats() * 4);
-                cudaFuncSetAttribute(k2_synthesize<8, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k2_smem_floats(256) * 4);
-                cudaFuncSetAttribute(k2_synthesize<8, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k2_smem_floats(256) * 4);
                 cudaFuncSetAttribute(k1n_magnitude<8, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k1n_smem_floats() * 4);
                 cudaFuncSetAttribute(k1d_analyze<8, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k1d_smem_bytes());
                 cudaFuncSetAttribute(k2d_synthesize<8, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k2d_smem_bytes());
@@ -903,12 +901,10 @@ int b200gate_create(const b200gate_params* p, b200gate_handle** out) {
                 cudaFuncSetAttribute(k2c_synthesize<8, kMaskU16Blend, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k2c_smem_bytes<kMaskU16Blend>());
                 cudaFuncSetAttribute(k2c_synthesize<8, kMaskF32, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, k2c_smem_bytes<kMaskF32>());
             });
-        cudaFuncSetAttribute(k1_analyze<8, float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, k1_smem_floats_staged() * 4);
         cudaFuncSetAttribute(k_smooth_f, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         cudaFuncSetAttribute(k_smooth_stream, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         for (int nfb = 1; nfb <= 12; ++nfb) smooth_box_dispatch(SmoothFArgs{}, nfb, dim3(1), 0, nullptr, true);
         cudaFuncSetAttribute(k1n_magnitude_2k, cudaFuncAttributeMaxDynamicSharedMemorySize, k1n2_smem_floats() * 4);
-        cudaFuncSetAttribute(k2_synthesize_2k, cudaFuncAttributeMaxDynamicSharedMemorySize, k22_smem_floats() * 4);
         cudaFuncSetAttribute(k2c_synthesize_2k, cudaFuncAttributeMaxDynamicSharedMemorySize, k2c2_smem_bytes());
         cudaFuncSetAttribute(k_smooth_generic, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
         for (int dt = 0; dt < 3; ++dt)
@@ -1332,13 +1328,12 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
     const size_t per_unit_2pass = (stat ? (size_t)g.T * kFW * 4 + (size_t)kFPad * 4 + (size_t)kFW * 4 + (size_t)num_unit_stride(g.T) * 2 + 64
                                         : 2 * (size_t)g.T * FP * 4 + 64) +
                                   (stat && torch_sem ? (size_t)g.T * kFPad * 4 + 2 * (size_t)kFPad * 4 : 0) + 2048;
-    // spectrum cache: k1 / k1n keep the packed spectrum of every frame pair so k2 does not re-transform
-    const int zpairs = (g.T + 1) / 2;
-    const bool use_zcache = !generic && !(p.path_flags & 2);
+    // spectrum cache of the tuned geometries: k1 / k1n keep the packed spectrum of every frame pair so k2 does not re-transform
     // (n_fft 2048: one half-length spectrum per frame; n_fft 1024: one packed spectrum per frame pair)
-    const size_t zunit = use_zcache ? (size_t)(two_k ? g.T : zpairs) * 1024 * sizeof(float2) : 0;
+    const int zpairs = (g.T + 1) / 2;
+    const size_t zunit = generic ? 0 : (size_t)(two_k ? g.T : zpairs) * 1024 * sizeof(float2);
     // dual kernels (gate_dual.cuh): two channels of a chunk per warp -- stationary numpy-surface gate, even channel count
-    const bool use_dual = use_zcache && stat && !torch_sem && native && (C % 2 == 0) && !(p.path_flags & 16);
+    const bool use_dual = !generic && stat && !torch_sem && native && (C % 2 == 0) && !(p.path_flags & 16);
     // general-geometry family: float64 spectrum, mask, scratch and synthesis frames of every unit
     const size_t g_tf = (size_t)g.T * (size_t)h->F, g_tw = (size_t)g.T * (size_t)h->g_W;
     const size_t per_unit_generic = g_tf * 16 + 2 * g_tf * 8 + g_tw * 8 + 2 * (size_t)h->F * 8 + 6 * 256;
@@ -1436,7 +1431,7 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
     float* d_tdb = (float*)(h->d_ws_buf + off_tdb);
     float* d_trow = (float*)(h->d_ws_buf + off_trow);
     float* d_tthr_self = (float*)(h->d_ws_buf + off_tthr);
-    float2* d_zcache = use_zcache ? (float2*)(h->d_ws_buf + off_z) : nullptr;
+    float2* d_zcache = generic ? nullptr : (float2*)(h->d_ws_buf + off_z);
     unsigned* d_bits = (unsigned*)(h->d_ws_buf + off_bits);
     unsigned* d_rowmax = (unsigned*)(h->d_ws_buf + off_rowmax);
     unsigned* d_rowflag = (unsigned*)(h->d_ws_buf + off_rowflag);
@@ -1665,7 +1660,6 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                 a1.g = g; a1.tb = tb; a1.x = xb; a1.bits = d_bits; a1.rowmax = d_rowmax; a1.cnt = h->d_cnt; a1.dbg = dbg;
                 a1.zcache = d_zcache; a1.zpairs = zpairs;
                 a1.z_lo = tf_lo; a1.z_hi = tf_hi + 1;           // k2 walks pairs (2j, 2j+1) of frames [tf_lo, tf_hi)
-                a1.stage_rows = ((p.path_flags & 8) && kdt == B200GATE_F32) ? 1 : 0;
                 {
                     long long want = (long long)h->num_sm * B200_K1_MINBLOCKS * kWarps * 4;
                     long long run = ((long long)nu * g.T + want - 1) / want;
@@ -1682,7 +1676,6 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                     K1dArgs ad{};
                     ad.g = g; ad.tb = tb; ad.x = xb; ad.bits = d_bits; ad.zd = (float4*)d_zcache; ad.zpairs = zpairs;
                     ad.z_lo = tf_lo; ad.z_hi = tf_hi + 1; ad.cnt = h->d_cnt; ad.need_rowmax = h->d_need_rowmax;
-                    if (getenv("B200GATE_DBG_NOCACHE_STORE")) ad.z_hi = 0;        // timing experiment only: results are wrong
                     ad.min_floor4 = (float)(4.0 * h->min_floor_amp * h->min_floor_amp);
                     ad.wa_max = h->wa_max; ad.dbg = dbg;
                     {
@@ -1700,15 +1693,9 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                     a1.guard = h->d_need_rowmax;
                     a1.zcache = nullptr;
                 }
-                if (a1.stage_rows) {
-                    auto kern_ = k1_analyze<8, float, true>;
+                B200_WITH_DTYPE(kdt, { auto kern_ = k1_analyze<8, T>;
                     B200_LAUNCH(kern_, dim3(grid_1d(items1, kWarps, h->num_sm * B200_K1_MINBLOCKS)), dim3(kThreads),
-                                k1_smem_floats_staged() * 4, st, a1);
-                } else {
-                    B200_WITH_DTYPE(kdt, { auto kern_ = k1_analyze<8, T>;
-                        B200_LAUNCH(kern_, dim3(grid_1d(items1, kWarps, h->num_sm * B200_K1_MINBLOCKS)), dim3(kThreads),
-                                    k1_smem_floats() * 4, st, a1); });
-                }
+                                k1_smem_floats() * 4, st, a1); });
                 B200_LAUNCH(k_rowfloor, dim3(grid_1d((long long)nu * kFW, 256, 1 << 30)), dim3(256), 0, st, nu,
                             (const unsigned*)d_rowmax, (const float*)h->d_floor4, d_rowflag, h->d_cnt);
             }
@@ -1750,7 +1737,7 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                 }
                 cudaEventRecord(h->stage_ev[4 * bi + 2], st);
                 K2Args a2{};
-                a2.g = g; a2.tb = tb; a2.x = xb; a2.y = yb; a2.num = d_num; a2.zcache = d_zcache; a2.zpairs = zpairs;
+                a2.g = g; a2.tb = tb; a2.y = yb; a2.num = d_num; a2.zcache = d_zcache; a2.zpairs = zpairs;
                 a2.pD = (float)(p.prop_decrease / D);
                 a2.one_minus_p = (float)(1.0 - p.prop_decrease);
                 a2.nt = nt;
@@ -1788,20 +1775,14 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                             B200_LAUNCH(kern2, dim3(grid_1d(itemsd, kDualWarpsK2, h->num_sm)), dim3(kDualWarpsK2 * 32),
                                         k2d_smem_bytes(), st, ad); });
                     }
-                } else if (use_zcache) {           // spectra kept by k1: bulk-staged synthesis (gate_synth.cuh)
-                    if (a2.one_minus_p != 0.f) {
-                        B200_WITH_DTYPE(kdt, { auto kern2 = k2c_synthesize<8, kMaskU16Blend, T>;
-                            B200_LAUNCH(kern2, dim3(grid_1d(items2, kWarps, resident)), dim3(kThreads),
-                                        k2c_smem_bytes<kMaskU16Blend>(), st, a2); });
-                    } else {
-                        B200_WITH_DTYPE(kdt, { auto kern2 = k2c_synthesize<8, kMaskU16, T>;
-                            B200_LAUNCH(kern2, dim3(grid_1d(items2, kWarps, resident)), dim3(kThreads),
-                                        k2c_smem_bytes<kMaskU16>(), st, a2); });
-                    }
-                } else {
-                    B200_WITH_DTYPE(kdt, { auto kern2 = k2_synthesize<8, false, T>;
+                } else if (a2.one_minus_p != 0.f) {       // spectra kept by k1: bulk-staged synthesis (gate_synth.cuh)
+                    B200_WITH_DTYPE(kdt, { auto kern2 = k2c_synthesize<8, kMaskU16Blend, T>;
                         B200_LAUNCH(kern2, dim3(grid_1d(items2, kWarps, resident)), dim3(kThreads),
-                                    k2_smem_floats(g.H) * 4, st, a2); });
+                                    k2c_smem_bytes<kMaskU16Blend>(), st, a2); });
+                } else {
+                    B200_WITH_DTYPE(kdt, { auto kern2 = k2c_synthesize<8, kMaskU16, T>;
+                        B200_LAUNCH(kern2, dim3(grid_1d(items2, kWarps, resident)), dim3(kThreads),
+                                    k2c_smem_bytes<kMaskU16>(), st, a2); });
                 }
                 cudaEventRecord(h->stage_ev[4 * bi + 3], st);
                 launches += 2;
@@ -1811,7 +1792,6 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                 Tables2 t2{};
                 t2.wa2 = h->d_wa2; t2.ws2 = h->d_ws2; t2.tw = h->d_tw; t2.w2k = h->d_w2k; t2.invn2 = h->d_invn2;
                 t2.ws_to_w = h->ws_to_w;
-                const int res2 = h->num_sm * 2;
                 cudaEventRecord(h->stage_ev[4 * bi + 0], st);
                 K1n2Args a1{};
                 a1.g = g; a1.tb = t2; a1.x = (const float*)xb; a1.mag = d_mag; a1.dbg = dbg;
@@ -1846,29 +1826,16 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                     sa.m0 = d_m0; sa.m2 = d_mag;
                     launch_smooth_float(sa, nf, nt, tf_lo, tf_hi, nu, p.path_flags, st);
                     cudaEventRecord(h->stage_ev[4 * bi + 2], st);
-                    if (use_zcache) {                  // spectra kept by k1n: bulk-staged synthesis (gate_synth_2k.cuh)
-                        K2c2Args ac{};
-                        ac.g = g; ac.tb = t2; ac.y = (float*)yb; ac.fmask = d_mag; ac.zcache = d_zcache; ac.dbg = dbg;
-                        const long long hops = h_hi - h_lo;
-                        long long want = (long long)h->num_sm * kK2c2Warps * 4;
-                        long long run = ((long long)nu * hops + want - 1) / want;
-                        ac.run = (int)std::max(16LL, std::min(128LL, run));
-                        ac.n_runs = (int)((hops + ac.run - 1) / ac.run);
-                        B200_LAUNCH(k2c_synthesize_2k, dim3(grid_1d((long long)nu * ac.n_runs, kK2c2Warps, h->num_sm)),
-                                    dim3(kK2c2Warps * 32), k2c2_smem_bytes(), st, ac);
-                    } else {
-                    K22Args a2{};
-                    a2.g = g; a2.tb = t2; a2.x = (const float*)xb; a2.y = (float*)yb; a2.fmask = d_mag; a2.dbg = dbg;
-                    {
-                        const long long hops = h_hi - h_lo;
-                        long long want = (long long)res2 * kWarps * 4;
-                        long long run = ((long long)nu * hops + want - 1) / want;
-                        a2.run = (int)std::max(16LL, std::min(128LL, run));
-                        a2.n_runs = (int)((hops + a2.run - 1) / a2.run);
-                    }
-                    B200_LAUNCH(k2_synthesize_2k, dim3(grid_1d((long long)nu * a2.n_runs, kWarps, res2)), dim3(kThreads),
-                                k22_smem_floats() * 4, st, a2);
-                    }
+                    // spectra kept by k1n: bulk-staged synthesis (gate_synth_2k.cuh)
+                    K2c2Args ac{};
+                    ac.g = g; ac.tb = t2; ac.y = (float*)yb; ac.fmask = d_mag; ac.zcache = d_zcache; ac.dbg = dbg;
+                    const long long hops = h_hi - h_lo;
+                    long long want = (long long)h->num_sm * kK2c2Warps * 4;
+                    long long run = ((long long)nu * hops + want - 1) / want;
+                    ac.run = (int)std::max(16LL, std::min(128LL, run));
+                    ac.n_runs = (int)((hops + ac.run - 1) / ac.run);
+                    B200_LAUNCH(k2c_synthesize_2k, dim3(grid_1d((long long)nu * ac.n_runs, kK2c2Warps, h->num_sm)),
+                                dim3(kK2c2Warps * 32), k2c2_smem_bytes(), st, ac);
                     cudaEventRecord(h->stage_ev[4 * bi + 3], st);
                     launches += 2;
                 }
@@ -1912,7 +1879,7 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                     }
                     cudaEventRecord(h->stage_ev[4 * bi + 2], st);
                     K2Args a2{};
-                    a2.g = g; a2.tb = tb; a2.x = xb; a2.y = yb; a2.fmask = d_mag; a2.zcache = d_zcache; a2.zpairs = zpairs;
+                    a2.g = g; a2.tb = tb; a2.y = yb; a2.fmask = d_mag; a2.zcache = d_zcache; a2.zpairs = zpairs;
                     a2.nt = nt;
                     a2.dbg = dbg;
                     {
@@ -1924,15 +1891,9 @@ int b200gate_run(b200gate_handle* h, const void* in, void* out, int dtype, int64
                         a2.run = (int)run;
                         a2.n_runs = (int)((hops + a2.run - 1) / a2.run);
                     }
-                    if (use_zcache) {
-                        B200_WITH_DTYPE(kdt, { auto kern2 = k2c_synthesize<8, kMaskF32, T>;
-                            B200_LAUNCH(kern2, dim3(grid_1d((long long)nu * a2.n_runs, kWarps, resident)), dim3(kThreads),
-                                        k2c_smem_bytes<kMaskF32>(), st, a2); });
-                    } else {
-                        B200_WITH_DTYPE(kdt, { auto kern2 = k2_synthesize<8, true, T>;
-                            B200_LAUNCH(kern2, dim3(grid_1d((long long)nu * a2.n_runs, kWarps, resident)), dim3(kThreads),
-                                        k2_smem_floats(g.H) * 4, st, a2); });
-                    }
+                    B200_WITH_DTYPE(kdt, { auto kern2 = k2c_synthesize<8, kMaskF32, T>;
+                        B200_LAUNCH(kern2, dim3(grid_1d((long long)nu * a2.n_runs, kWarps, resident)), dim3(kThreads),
+                                    k2c_smem_bytes<kMaskF32>(), st, a2); });
                     cudaEventRecord(h->stage_ev[4 * bi + 3], st);
                     launches += 2;
                 }

@@ -20,8 +20,8 @@
 //   k_rowfloor    top_db floor:  max_t dB - top_db > thresh  <=>  lift the whole row
 //   k_smooth      separable triangular smoothing of the binary mask in exact integer arithmetic
 //                 (the reference's FFT convolution approximates exactly these rationals)
-//   k2_synthesize frames -> FFT -> mask apply on the packed spectrum -> inverse FFT -> window ->
-//                 overlap-add in registers -> normalise -> store the chunk centre
+//   k2c / k2d     synthesis (gate_synth.cuh, gate_dual.cuh): the spectra k1 kept -> mask apply on the packed
+//                 spectrum -> inverse FFT -> window -> overlap-add in registers -> normalise -> store the chunk centre
 #pragma once
 #include "warp_fft.cuh"
 
@@ -180,40 +180,6 @@ __device__ __forceinline__ float load_frame_pair(float (&re)[32], float (&im)[32
     return pack_frame_pair<HR>(re, im, xr, s_wa, lane, vb);
 }
 
-// Asynchronous global -> shared copies (LDGSTS): the next frame pair's cached spectrum is requested one whole
-// iteration before it is needed and costs no registers while in flight.
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-#ifdef B200_CUSIM_BUILD
-    memcpy(smem_dst, gmem_src, 16);
-#else
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(gmem_src));
-#endif
-}
-__device__ __forceinline__ void cp_async4(void* smem_dst, const void* gmem_src) {
-#ifdef B200_CUSIM_BUILD
-    memcpy(smem_dst, gmem_src, 4);
-#else
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(sa), "l"(gmem_src));
-#endif
-}
-__device__ __forceinline__ void cp_async_commit_wait_all() {
-#ifndef B200_CUSIM_BUILD
-    asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-#endif
-}
-__device__ __forceinline__ void cp_async_commit() {
-#ifndef B200_CUSIM_BUILD
-    asm volatile("cp.async.commit_group;" ::: "memory");
-#endif
-}
-__device__ __forceinline__ void cp_async_wait_all() {
-#ifndef B200_CUSIM_BUILD
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-#endif
-}
-
 #ifdef B200_CUSIM_BUILD
 #define B200_NOINLINE __attribute__((noinline))
 #else
@@ -260,15 +226,11 @@ struct K1Args {
     int z_lo, z_hi;            // only frames [z_lo, z_hi) are read back by k2 (chunk centre + halo): the rest is not stored
     const unsigned* guard;     // optional device flag: when given and zero the kernel returns at once (it is then the
                                // row-maximum fallback behind k1d_analyze, gate_dual.cuh)
-    int stage_rows;            // set for the k1_analyze<.., true> instantiation (path_flags bit 3, float32 rows): the NEXT
-                               // pair's sample rows stream into shared memory (cp.async) behind the current pair's transform
 };
 
 constexpr int k1_smem_floats() { return kN + 2 * kN + 2 * kFPad + kWarps * kExchFloats + kWarps * 2 * kFW + 8; }
-constexpr int kStageFloats = 32 * (32 + 8);          // one pair's rows: 40 x 32 samples
-constexpr int k1_smem_floats_staged() { return k1_smem_floats() + kWarps * kStageFloats; }
 
-template <int HR, typename T, bool STAGE = false>
+template <int HR, typename T>
 __global__ void __launch_bounds__(kThreads, B200_K1_MINBLOCKS) k1_analyze(const K1Args a) {
     if (a.guard && *a.guard == 0u) return;
     B200_DYN_SMEM(float, smem);
@@ -278,7 +240,6 @@ __global__ void __launch_bounds__(kThreads, B200_K1_MINBLOCKS) k1_analyze(const 
     float* s_gco = s_thr4 + kFPad;
     float* s_tiles = s_gco + kFPad;
     unsigned* s_amb_all = reinterpret_cast<unsigned*>(s_tiles + kWarps * kExchFloats);
-    float* s_stage_all = reinterpret_cast<float*>(s_amb_all + kWarps * 2 * kFW + 8);    // only when a.stage_rows
     for (int i = threadIdx.x; i < kN; i += kThreads) {
         s_wa[i] = a.tb.wa[i];
         s_tw[i] = a.tb.tw[i];
@@ -311,45 +272,11 @@ __global__ void __launch_bounds__(kThreads, B200_K1_MINBLOCKS) k1_analyze(const 
 #pragma unroll
         for (int q = 0; q < kFW; ++q) mx[q] = 0.f;
 
-        // staged rows: request pair t's 40 rows (float32, interior of the chunk and the recording) into this
-        // warp's 5 KB buffer; 16-byte copies when the first row is 16-byte aligned, else one word per lane and row
-        float* sbuf = s_stage_all + warp * kStageFloats;
-        auto stage_rows = [&](int tt) -> bool {
-            if (!STAGE || sizeof(T) != 4) return false;       // compile-time: the default instantiation carries none of this
-            const long long bb = (long long)tt * H - kN / 2;
-            if (!pair_window_interior<HR>(bb, i1, g.Lp, g.n_total)) return false;
-            const char* src = reinterpret_cast<const char*>(xrow + i1 + bb);
-            char* dst = reinterpret_cast<char*>(sbuf);
-            if ((reinterpret_cast<unsigned long long>(src) & 15ull) == 0) {
-#pragma unroll
-                for (int j = 0; j < (32 + HR) / 4; ++j) cp_async16(dst + (lane + 32 * j) * 16, src + (lane + 32 * j) * 16);
-            } else {
-#pragma unroll
-                for (int r = 0; r < 32 + HR; ++r) cp_async4(dst + (lane + 32 * r) * 4, src + (lane + 32 * r) * 4);
-            }
-            cp_async_commit();
-            return true;
-        };
-        bool staged = STAGE && stage_rows(t0);
-
         for (int t = t0; t < t1; t += 2) {
             const bool vb = (t + 1 < t1);
             const long long base = (long long)t * H - kN / 2;
             float re[32], im[32];
-            float e;
-            if (STAGE && staged) {                            // warp-uniform
-                float xr[32 + HR];
-                cp_async_wait_all();
-                __syncwarp();
-#pragma unroll
-                for (int r = 0; r < 32 + HR; ++r) xr[r] = sbuf[32 * r + lane];
-                __syncwarp();
-                staged = (t + 2 < t1) && stage_rows(t + 2);   // the next pair streams in behind this pair's transform
-                e = pack_frame_pair<HR>(re, im, xr, s_wa, lane, vb);
-            } else {
-                if (STAGE) staged = (t + 2 < t1) && stage_rows(t + 2);
-                e = load_frame_pair<HR>(re, im, xrow, base, i1, g.Lp, g.n_total, s_wa, lane, vb);
-            }
+            const float e = load_frame_pair<HR>(re, im, xrow, base, i1, g.Lp, g.n_total, s_wa, lane, vb);
             const float S = sqrtf(warp_sum(e));
             warp_fft1024(re, im, tile, s_tw, lane);
             if (a.zcache && t >= a.z_lo && t < a.z_hi) {      // warp-uniform
@@ -692,12 +619,11 @@ __global__ void __launch_bounds__(kSmoothThreads, 3) k_smooth_packed(const Smoot
 }
 
 // =============================================================================================
-// k2: synthesis.
+// k2: synthesis (k2c_synthesize, gate_synth.cuh).
 // =============================================================================================
 struct K2Args {
     Geom g;
     Tables tb;
-    const void* x;                 // caller dtype (kernel template T)
     void* y;                       // [C][out_stride], caller dtype
     const unsigned short* num;     // [n_units][T][FPad] integer mask numerators (stationary)
     const float* fmask;            // [n_units][T][FPad] final float masks (non-stationary)
@@ -707,11 +633,9 @@ struct K2Args {
     int run;                       // output hops per work item
     int n_runs;
     DebugTap dbg;
-    const float2* zcache;          // optional: spectra stored by k1 / k1n (frames then are not re-transformed)
+    const float2* zcache;          // packed spectra of the frame pairs, stored by k1 / k1n
     int zpairs;
 };
-
-constexpr int k2_smem_floats(int H) { return 2 * kN + 2 * kN + H + kFPad + kWarps * kExchFloats + 8 + kWarps * 2 * kN; }
 
 // time edge factor of the zero-padded smoothing: sum of the triangle taps that stay inside [0, T)
 __device__ __forceinline__ float time_edge(int t, int T, int nt) {
@@ -721,249 +645,14 @@ __device__ __forceinline__ float time_edge(int t, int T, int nt) {
     return (float)s / (float)((nt + 1) * (nt + 1));
 }
 
-template <int HR, bool FMASK, typename T>
-__global__ void __launch_bounds__(kThreads, 3) k2_synthesize(const K2Args a) {
-    constexpr int NH = 32 / HR;             // frames overlapping one hop (win / hop)
-    B200_DYN_SMEM(float, smem);
-    const Geom& g = a.g;
-    const int H = g.H;
-    float* s_wa = smem;
-    float* s_ws = smem + kN;
-    float2* s_tw = reinterpret_cast<float2*>(smem + 2 * kN);
-    float* s_invn = smem + 4 * kN;
-    float* s_ef = s_invn + H;
-    float* s_tiles = s_ef + kFPad;
-    for (int i = threadIdx.x; i < kN; i += kThreads) {
-        s_wa[i] = a.tb.wa[i];
-        s_ws[i] = a.tb.ws[i];
-        s_tw[i] = a.tb.tw[i];
-    }
-    for (int i = threadIdx.x; i < H; i += kThreads) s_invn[i] = a.tb.invn[i];
-    for (int i = threadIdx.x; i < kFPad; i += kThreads) s_ef[i] = a.tb.ef[i];
-    __syncthreads();
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    float* tile = s_tiles + warp * kExchFloats;
-    // per-warp staging buffer of one cached spectrum (8 KB), 16-byte aligned behind the tiles
-    float2* zbuf = reinterpret_cast<float2*>(s_tiles + kWarps * kExchFloats + 8) + warp * kN;
-    const int pl = (32 - lane) & 31;
-    const long long n_items = (long long)g.n_units * a.n_runs;
-    const bool blend = (a.one_minus_p != 0.f);
-
-    for (long long item = (long long)blockIdx.x * kWarps + warp; item < n_items;
-         item += (long long)gridDim.x * kWarps) {
-        const int ul = (int)(item / a.n_runs);
-        const int run = (int)(item - (long long)ul * a.n_runs);
-        const int u = g.u0 + ul;
-        const int ic = u / g.C, c = u - ic * g.C;
-        const long long i1 = (long long)ic * g.step - g.pad;
-        long long out_len = g.n_total - (long long)ic * g.step;
-        if (out_len > g.step) out_len = g.step;
-        // valid chunk-local output range [pad, jp_hi), in padded (frame) coordinates + N/2
-        long long jp_hi = g.pad + out_len;
-        const long long sig_len = (long long)(g.T - 1) * H;          // istft output length
-        if (jp_hi > sig_len) jp_hi = sig_len;                        // beyond it the reference leaves zeros
-        if (jp_hi <= g.pad) continue;
-        const long long jlo = g.pad + kN / 2, jhi = jp_hi + kN / 2;
-        const int h_lo = (int)(jlo / H), h_hi = (int)((jhi + H - 1) / H);
-        const int hs = h_lo + run * a.run;
-        const int he = min(hs + a.run, h_hi);
-        if (hs >= he) continue;
-        int t_start = max(0, hs - (NH - 1));
-        if (a.zcache) t_start &= ~1;                 // k1 packed frames (2j, 2j+1): walk the same pairs
-        const int t_last = min(he - 1, g.T - 1);
-        const T* xrow = static_cast<const T*>(a.x) + (long long)c * g.in_stride;
-        T* yrow = static_cast<T*>(a.y) + (long long)c * g.out_stride;
-        const unsigned short* mrow = FMASK ? nullptr : a.num + (long long)ul * num_unit_stride(g.T);
-        const float* frow = FMASK ? a.fmask + (long long)ul * g.T * kFPad : nullptr;
-
-        float acc[32 + HR];
-#pragma unroll
-        for (int r = 0; r < 32 + HR; ++r) acc[r] = 0.f;
-
-        auto stage_spectrum = [&](int tt) {            // request pair (tt, tt+1)'s spectrum into zbuf
-            const char* src = reinterpret_cast<const char*>(a.zcache + ((long long)ul * a.zpairs + (tt >> 1)) * 1024);
-            char* dst = reinterpret_cast<char*>(zbuf);
-#pragma unroll
-            for (int j = 0; j < 16; ++j) cp_async16(dst + (lane + 32 * j) * 16, src + (lane + 32 * j) * 16);
-            cp_async_commit();
-        };
-        if (a.zcache && t_start <= t_last) stage_spectrum(t_start);
-
-        for (int t = t_start; t < he; t += 2) {
-            const bool va = (t <= t_last), vb = (t + 1 <= t_last);
-            if (va) {                                   // vb implies va
-                const long long base = (long long)t * H - kN / 2;
-                float re[32], im[32];
-                if (!a.zcache) load_frame_pair<HR>(re, im, xrow, base, i1, g.Lp, g.n_total, s_wa, lane, vb);
-                const long long offA = (long long)t * kFPad, offB = (long long)(vb ? t + 1 : t) * kFPad;
-                // the masks of this pair are requested now, a whole FFT before the apply step needs them
-                float mka[kFW], mkb[FMASK ? kFW : 1];         // uint16 numerators travel packed two per register
-#pragma unroll
-                for (int q = 0; q < kFW; ++q) {
-                    const int k = lane + 32 * q;                         // < FPad, rows are padded
-                    if (FMASK) {
-                        mka[q] = frow[offA + k];
-                        mkb[FMASK ? q : 0] = frow[offB + k];
-                    } else {
-                        mka[q] = __uint_as_float((unsigned)mrow[num_index(t, k)] | ((unsigned)mrow[num_index(vb ? t + 1 : t, k)] << 16));
-                    }
-                }
-                float eta = 0.f, etb = 0.f;
-                if (!FMASK && blend) {
-                    eta = a.one_minus_p * time_edge(t, g.T, a.nt);
-                    etb = a.one_minus_p * time_edge(t + 1, g.T, a.nt);
-                }
-                if (a.dbg.ul == ul) {                        // parity tap (tests): the masks this pair applies
-#pragma unroll 1
-                    for (int k = lane; k < kF; k += 32) {
-                        float ma, mb;
-                        if (FMASK) {
-                            ma = frow[offA + k];
-                            mb = frow[offB + k];
-                        } else {
-                            ma = fmaf((float)mrow[num_index(t, k)], a.pD, eta * s_ef[k]);
-                            mb = fmaf((float)mrow[num_index(vb ? t + 1 : t, k)], a.pD, etb * s_ef[k]);
-                        }
-                        a.dbg.mask[(long long)t * kF + k] = ma;
-                        if (vb) a.dbg.mask[(long long)(t + 1) * kF + k] = mb;
-                    }
-                }
-                // phase 0: forward FFT + mask apply; phase 1: inverse FFT.  One copy of the FFT code
-                // serves both: the apply step leaves Z' with real/imaginary parts exchanged and in
-                // natural slot order, so ifft(Z') = swap(fft(swap(Z'))) is the very same call.
-                const bool cached = a.zcache != nullptr;
-                if (cached) {                                // the forward transform of this pair was done by k1
-                    cp_async_wait_all();
-                    __syncwarp();
-#pragma unroll
-                    for (int q = 0; q < 32; ++q) {
-                        const float2 v = zbuf[32 * q + lane];
-                        re[brev5(q)] = v.x;
-                        im[brev5(q)] = v.y;
-                    }
-                    __syncwarp();
-                    if (t + 2 <= t_last) stage_spectrum(t + 2);   // next pair streams in behind this pair's math
-                }
-#pragma unroll 1
-                for (int ph = 0; ph < 2; ++ph) {
-                    if (!(cached && ph == 0)) warp_fft1024(re, im, tile, s_tw, lane);
-                    if (ph == 0) {
-#pragma unroll
-                        for (int q = 0; q < kFW; ++q) {
-                            const int sA = brev5(q), sP = brev5(31 - q), s0 = brev5((32 - q) & 31);
-                            const int k = lane + 32 * q;
-                            float ma, mb;
-                            if (FMASK) {
-                                ma = mka[q];
-                                mb = mkb[FMASK ? q : 0];
-                            } else {
-                                const unsigned pk = __float_as_uint(mka[q]);
-                                ma = fmaf(u16lo_to_float(pk), a.pD, eta * s_ef[k]);
-                                mb = fmaf(u16hi_to_float(pk), a.pD, etb * s_ef[k]);
-                            }
-                            if (!vb) mb = 0.f;
-                            const float s = 0.5f * (ma + mb), d = 0.5f * (ma - mb);
-                            const float zr = re[sA], zi = im[sA];
-                            if (q < 16) {
-                                float pr = __shfl_sync(0xffffffffu, re[sP], pl);
-                                float pi = __shfl_sync(0xffffffffu, im[sP], pl);
-                                if (lane == 0) { pr = re[s0]; pi = im[s0]; }
-                                // Z'[k] = s Z[k] + d conj(Z[N-k]);  Z'[N-k] = s Z[N-k] + d conj(Z[k])
-                                const float own_r = fmaf(d, pr, s * zr), own_i = fmaf(-d, pi, s * zi);
-                                const float oth_r = fmaf(d, zr, s * pr), oth_i = fmaf(-d, zi, s * pi);
-                                const float nr = __shfl_sync(0xffffffffu, oth_r, pl);
-                                const float ni = __shfl_sync(0xffffffffu, oth_i, pl);
-                                re[sA] = own_r;
-                                im[sA] = own_i;
-                                if (lane != 0) { re[sP] = nr; im[sP] = ni; }
-                                else if (q != 0) { re[s0] = oth_r; im[s0] = oth_i; }
-                            } else if (lane == 0) {                      // bin N/2 mirrors onto itself
-                                re[sA] = fmaf(d, zr, s * zr);
-                                im[sA] = fmaf(-d, zi, s * zi);
-                            }
-                        }
-                        // brev slots -> natural slots with re <-> im exchanged, in place (2-cycles of brev5)
-#pragma unroll
-                        for (int q = 0; q < 32; ++q) {
-                            const int b = brev5(q);
-                            if (b == q) {
-                                const float tr = re[q];
-                                re[q] = im[q];
-                                im[q] = tr;
-                            } else if (q < b) {
-                                const float t1 = re[q], t2 = im[q];
-                                re[q] = im[b];
-                                im[q] = re[b];
-                                re[b] = t2;
-                                im[b] = t1;
-                            }
-                        }
-                    }
-                }
-                // now im = N a'[n], re = N b'[n] (n = lane + 32 q) at slot brev5(q)
-#pragma unroll
-                for (int q = 0; q < 32; ++q) {
-                    const float w = s_ws[lane + 32 * q];
-                    acc[q] = fmaf(im[brev5(q)], w, acc[q]);
-                    acc[q + HR] = fmaf(re[brev5(q)], w, acc[q + HR]);
-                }
-            }
-            // hops t and t+1 are now complete (all frames <= t+1 have been added)
-            {
-                const long long jp0 = (long long)t * H - kN / 2;             // chunk-local index of row 0, lane 0
-                if (t >= hs && t + 1 < he && t >= NH - 1 && t + 1 <= g.T - 1 && jp0 >= g.pad &&
-                    jp0 + 2 * H <= jp_hi) {
-                    // both hops interior and fully inside the chunk centre: 2*HR coalesced row stores
-                    T* dst = yrow + i1 + jp0 + lane;
-#pragma unroll
-                    for (int r = 0; r < 2 * HR; ++r) dst[32 * r] = st_cast<T>(acc[r] * s_invn[(r % HR) * 32 + lane]);
-                } else {
-#pragma unroll 1
-                    for (int r = 0; r < 2 * HR; ++r) {
-                        float v = 0.f;
-#pragma unroll
-                        for (int rr = 0; rr < 2 * HR; ++rr)
-                            if (rr == r) v = acc[rr];
-                        const int hop = t + r / HR;
-                        if (hop < hs || hop >= he) continue;
-                        const int ro = (r % HR) * 32 + lane;
-                        const long long jp = (long long)hop * H + ro - kN / 2;   // chunk-local output index
-                        if (jp < g.pad || jp >= jp_hi) continue;
-                        float inv;
-                        if (hop >= NH - 1 && hop <= g.T - 1) {
-                            inv = s_invn[ro];
-                        } else {                                                  // first / last hops
-                            float nrm = 0.f;
-                            for (int i = 0; i < NH; ++i) {
-                                const int tf = hop - i;
-                                if (tf >= 0 && tf <= g.T - 1) {
-                                    const float w = s_ws[i * H + ro] * a.tb.ws_to_w;
-                                    nrm = fmaf(w, w, nrm);
-                                }
-                            }
-                            inv = nrm > 1e-10f ? 1.0f / nrm : 1.0f;
-                        }
-                        yrow[i1 + jp] = st_cast<T>(v * inv);
-                    }
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < 32 - HR; ++r) acc[r] = acc[r + 2 * HR];
-#pragma unroll
-            for (int r = 32 - HR; r < 32 + HR; ++r) acc[r] = 0.f;
-        }
-    }
-}
-
-
 // =============================================================================================
 // Non-stationary gate (nonstationary.py:47-97).
 //   k1n_magnitude  frames -> FFT -> |X|                         [n_units][T][FPad] float32
 //   k_iir_sigmoid  filtfilt([b],[1,b-1]) along time per bin (forward sweep started at x[0], backward
 //                  sweep over the forward output started at its last value -- nonstationary.py:106-115),
 //                  then sigmoid(((|X| - S)/S - n_mult) * slope)  (spectralgate/utils.py:4-8)
-//   k_smooth_f     separable triangular smoothing (zero padded), then  m * p + (1 - p)
+//   k_smooth_box   separable triangular smoothing (zero padded), then  m * p + (1 - p); k_smooth_stream (nf > 12)
+//                  and k_smooth_f (time extent too long for shared memory) are its fallbacks
 // =============================================================================================
 struct K1nArgs {
     Geom g;
@@ -1235,10 +924,11 @@ __global__ void __launch_bounds__(256) k_smooth_f(const SmoothFArgs a) {
     }
 }
 
-// Streaming form of the same smoothing (the one that normally runs; k_smooth_f above is kept as its tile-based
-// cross-check).  A CTA walks a strip of frames of one unit; thread i owns bins i, i+G, i+2G, i+3G (G = FPad/4, so every
-// shared-memory access of a warp is 32 consecutive floats): the last 2 nt + 1 mask rows live in a ring of thread-private
-// columns (no barrier needed to refill it), the time-direction triangle is taken straight from the ring, the
+// Streaming form of the same smoothing (it runs where the box form below does not apply, e.g. nf > 12; k_smooth_f
+// above serves rings too large for shared memory).  A CTA walks a strip of frames of one unit; thread i owns bins
+// i, i+G, i+2G, i+3G (G = FPad/4, so every shared-memory access of a warp is 32 consecutive floats): the last
+// 2 nt + 1 mask rows live in a ring of thread-private columns (no barrier needed to refill it), the time-direction
+// triangle is taken straight from the ring, the
 // frequency-direction triangle from one zero-haloed row -- two barriers per frame, every mask value read from HBM
 // once per strip and written once.
 inline size_t smooths_smem_bytes(int FPad, int nf, int nt) { return ((size_t)(2 * nt + 1) * FPad + FPad + 2 * nf + 8) * 4; }

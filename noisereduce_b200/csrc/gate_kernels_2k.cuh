@@ -149,192 +149,4 @@ __global__ void __launch_bounds__(kThreads, 3) k1n_magnitude_2k(const K1n2Args a
     }
 }
 
-struct K22Args {
-    Geom g;
-    Tables2 tb;
-    const float* x;
-    float* y;
-    const float* fmask;        // [n_units][T][FPad2] final multiplicative masks
-    int run, n_runs;           // output hops per work item
-    DebugTap dbg;              // mask: [T][F2]
-};
-
-constexpr int k22_smem_floats() { return k2k_table_floats() + 2 * 1024 + 2 * 256 + kWarps * kExchFloats; }
-
-__global__ void __launch_bounds__(kThreads, 2) k2_synthesize_2k(const K22Args a) {
-    constexpr int HR = 8, NH = 4;
-    B200_DYN_SMEM(float, smem);
-    float2* s_wa2 = reinterpret_cast<float2*>(smem);
-    float2* s_tw = reinterpret_cast<float2*>(smem + 2048);
-    float2* s_w2k = reinterpret_cast<float2*>(smem + 4096);
-    float2* s_ws2 = reinterpret_cast<float2*>(smem + k2k_table_floats());
-    float2* s_invn2 = s_ws2 + 1024;
-    float* s_tiles = smem + k2k_table_floats() + 2 * 1024 + 2 * 256;
-    for (int i = threadIdx.x; i < 1024; i += kThreads) {
-        s_wa2[i] = a.tb.wa2[i];
-        s_tw[i] = a.tb.tw[i];
-        s_ws2[i] = a.tb.ws2[i];
-    }
-    for (int i = threadIdx.x; i < kFPad2; i += kThreads) s_w2k[i] = (i < kF2) ? a.tb.w2k[i] : make_float2(0.f, 0.f);
-    for (int i = threadIdx.x; i < 256; i += kThreads) s_invn2[i] = a.tb.invn2[i];
-    __syncthreads();
-
-    const Geom& g = a.g;
-    const int H = g.H;                                   // 512
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    float* tile = s_tiles + warp * kExchFloats;
-    const int pl = (32 - lane) & 31;
-    const long long n_items = (long long)g.n_units * a.n_runs;
-
-    for (long long item = (long long)blockIdx.x * kWarps + warp; item < n_items;
-         item += (long long)gridDim.x * kWarps) {
-        const int ul = (int)(item / a.n_runs);
-        const int run = (int)(item - (long long)ul * a.n_runs);
-        const int u = g.u0 + ul;
-        const int ic = u / g.C, c = u - ic * g.C;
-        const long long i1 = (long long)ic * g.step - g.pad;
-        long long out_len = g.n_total - (long long)ic * g.step;
-        if (out_len > g.step) out_len = g.step;
-        long long jp_hi = g.pad + out_len;
-        const long long sig_len = (long long)(g.T - 1) * H;
-        if (jp_hi > sig_len) jp_hi = sig_len;
-        if (jp_hi <= g.pad) continue;
-        const long long jlo = g.pad + kN2 / 2, jhi = jp_hi + kN2 / 2;
-        const int h_lo = (int)(jlo / H), h_hi = (int)((jhi + H - 1) / H);
-        const int hs = h_lo + run * a.run;
-        const int he = min(hs + a.run, h_hi);
-        if (hs >= he) continue;
-        const int t_start = max(0, hs - (NH - 1));
-        const int t_last = min(he - 1, g.T - 1);
-        const float* xrow = a.x + (long long)c * g.in_stride;
-        float* yrow = a.y + (long long)c * g.out_stride;
-        const float* frow = a.fmask + (long long)ul * g.T * kFPad2;
-
-        float acc_e[32], acc_o[32];                      // even / odd samples of the overlap-add window
-#pragma unroll
-        for (int r = 0; r < 32; ++r) { acc_e[r] = 0.f; acc_o[r] = 0.f; }
-
-        for (int t = t_start; t < he; ++t) {
-            if (t <= t_last) {
-                const long long base = (long long)t * H - kN2 / 2;
-                float re[32], im[32];
-                load_frame_2k(re, im, xrow, base, i1, g.Lp, g.n_total, s_wa2, lane);
-                const float* mrow = frow + (long long)t * kFPad2;
-                if (a.dbg.ul == ul) {
-#pragma unroll 1
-                    for (int k = lane; k < kF2; k += 32) a.dbg.mask[(long long)t * kF2 + k] = mrow[k];
-                }
-#pragma unroll 1
-                for (int ph = 0; ph < 2; ++ph) {
-                    warp_fft1024(re, im, tile, s_tw, lane);
-                    if (ph == 0) {
-#pragma unroll
-                        for (int q = 0; q < 17; ++q) {
-                            const int sA = brev5(q), sP = brev5(31 - q), s0 = brev5((32 - q) & 31);
-                            const int k = lane + 32 * q;                       // <= 543 < FPad2
-                            const float zr = re[sA], zi = im[sA];
-                            float pr, pi;
-                            if (q < 16) {
-                                pr = __shfl_sync(0xffffffffu, re[sP], pl);
-                                pi = __shfl_sync(0xffffffffu, im[sP], pl);
-                                if (lane == 0) { pr = re[s0]; pi = im[s0]; }
-                            } else {
-                                pr = zr; pi = zi;                              // only lane 0 (k = 512) matters
-                            }
-                            const float m = mrow[k];
-                            const float mp = mrow[(1024 - k) & 2047];          // k' = 1024-k (>= 481 for q = 16 lanes)
-                            const float Er = 0.5f * (zr + pr), Ei = 0.5f * (zi - pi);
-                            const float Or = 0.5f * (zi + pi), Oi = 0.5f * (pr - zr);
-                            const float2 W = s_w2k[k];
-                            const float Tr = fmaf(-Oi, W.y, Or * W.x), Ti = fmaf(Or, W.y, Oi * W.x);
-                            // P = X[k] = E + T,  Q = conj X[1024-k] = E - T;  masks applied to X[k], X[1024-k]
-                            const float Pr = m * (Er + Tr), Pi = m * (Ei + Ti);
-                            const float Qr = mp * (Er - Tr), Qi = mp * (Ei - Ti);
-                            const float Epr = 0.5f * (Pr + Qr), Epi = 0.5f * (Pi + Qi);
-                            const float Tpr = 0.5f * (Pr - Qr), Tpi = 0.5f * (Pi - Qi);
-                            // V = conj(W) T'   (W = (W.x, W.y) with W.y = -sin)
-                            const float Vr = fmaf(Tpi, W.y, Tpr * W.x), Vi = fmaf(-Tpr, W.y, Tpi * W.x);
-                            const float own_r = Epr - Vi, own_i = Epi + Vr;    // Z'[k]      = E' + i V
-                            const float oth_r = Epr + Vi, oth_i = Vr - Epi;    // Z'[1024-k] = conj(E') + i conj(V)
-                            if (q < 16) {
-                                const float nr = __shfl_sync(0xffffffffu, oth_r, pl);
-                                const float ni = __shfl_sync(0xffffffffu, oth_i, pl);
-                                re[sA] = own_r;
-                                im[sA] = own_i;
-                                if (lane != 0) { re[sP] = nr; im[sP] = ni; }
-                                else if (q != 0) { re[s0] = oth_r; im[s0] = oth_i; }
-                            } else if (lane == 0) {
-                                re[sA] = own_r;
-                                im[sA] = own_i;
-                            }
-                        }
-                        // brev slots -> natural slots with re <-> im exchanged, in place
-#pragma unroll
-                        for (int q = 0; q < 32; ++q) {
-                            const int b = brev5(q);
-                            if (b == q) {
-                                const float tr = re[q];
-                                re[q] = im[q];
-                                im[q] = tr;
-                            } else if (q < b) {
-                                const float t1 = re[q], t2 = im[q];
-                                re[q] = im[b];
-                                im[q] = re[b];
-                                re[b] = t2;
-                                im[b] = t1;
-                            }
-                        }
-                    }
-                }
-                // now im = 1024 * y[2m], re = 1024 * y[2m+1]  (m = lane + 32 q) at slot brev5(q)
-#pragma unroll
-                for (int q = 0; q < 32; ++q) {
-                    const float2 w = s_ws2[lane + 32 * q];
-                    acc_e[q] = fmaf(im[brev5(q)], w.x, acc_e[q]);
-                    acc_o[q] = fmaf(re[brev5(q)], w.y, acc_o[q]);
-                }
-            }
-            // hop t is complete: rows 0..7 (pairs) = samples [t*512, (t+1)*512)
-            if (t >= hs) {
-                const long long jp0 = (long long)t * H - kN2 / 2;          // chunk-local index of row 0, pair 0
-                float* d0 = yrow + i1 + jp0 + 2 * lane;
-                if (t >= NH - 1 && t <= g.T - 1 && jp0 >= g.pad && jp0 + H <= jp_hi &&
-                    ((reinterpret_cast<uintptr_t>(d0) & 7) == 0)) {
-#pragma unroll
-                    for (int r = 0; r < HR; ++r) {
-                        const float2 inv = s_invn2[r * 32 + lane];
-                        *reinterpret_cast<float2*>(d0 + 64 * r) = make_float2(acc_e[r] * inv.x, acc_o[r] * inv.y);
-                    }
-                } else {
-#pragma unroll
-                    for (int r = 0; r < HR; ++r) {
-#pragma unroll
-                        for (int par = 0; par < 2; ++par) {
-                            const int ro = r * 64 + 2 * lane + par;         // sample offset within the hop
-                            const long long jp = jp0 + ro;
-                            if (jp < g.pad || jp >= jp_hi) continue;
-                            float nrm = 0.f;
-                            for (int i = 0; i < NH; ++i) {
-                                const int tf = t - i;
-                                if (tf >= 0 && tf <= g.T - 1) {
-                                    const int n = i * H + ro;               // window index of this sample in frame tf
-                                    const float2 wp = s_ws2[n >> 1];
-                                    const float w = ((n & 1) ? wp.y : wp.x) * a.tb.ws_to_w;
-                                    nrm = fmaf(w, w, nrm);
-                                }
-                            }
-                            const float inv = nrm > 1e-10f ? 1.0f / nrm : 1.0f;
-                            yrow[i1 + jp] = (par ? acc_o[r] : acc_e[r]) * inv;
-                        }
-                    }
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < 32 - HR; ++r) { acc_e[r] = acc_e[r + HR]; acc_o[r] = acc_o[r + HR]; }
-#pragma unroll
-            for (int r = 32 - HR; r < 32; ++r) { acc_e[r] = 0.f; acc_o[r] = 0.f; }
-        }
-    }
-}
-
 }  // namespace b200

@@ -1,5 +1,5 @@
 // gate_synth_2k.cuh -- k2c_synthesize_2k: synthesis of the n_fft = 2048 family (BASELINE.json config 3) from the
-// spectra k1n_magnitude_2k kept, instead of transforming every frame a second time (k2_synthesize_2k).
+// spectra k1n_magnitude_2k kept, so that no frame is transformed a second time.
 //
 // Reference semantics (paths relative to /root/reference): mask apply at noisereduce/spectralgate/nonstationary.py:87,
 // scipy.signal.istft as called at nonstationary.py:90-96, chunk centre written back at base.py:150.

@@ -1,7 +1,6 @@
 """A/B of the config-3 (non-stationary, n_fft 2048, 64 ch x 10 min @ 48 kHz) kernel variants on one B200: step time, stage
 times from the library, and agreement of the outputs.   python scripts/ab_config3.py [flags ...]
-path_flags: 0 default | 128 tap-loop smoothing (k_smooth_stream) | 16 one frame per warp in the analysis (k1n_magnitude_2k)
-            | 2 no spectrum cache (k2_synthesize_2k re-transforms) | 64 follower stores its forward sweep"""
+path_flags: 0 default | 128 tap-loop smoothing (k_smooth_stream) | 64 follower stores its forward sweep"""
 import json
 import os
 import sys
@@ -12,7 +11,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bench import synth_device, SR, C_PER_GPU  # noqa: E402
 from noisereduce_b200.device import DeviceGate  # noqa: E402
 
-flags = [a for a in sys.argv[1:]] or ["0", "128", "2", "64"]     # an argument "v:NAME" times libb200gate_NAME.so (scripts/build_variant.py) with path_flags 0
+flags = [a for a in sys.argv[1:]] or ["0", "128", "64"]     # an argument "v:NAME" times libb200gate_NAME.so (scripts/build_variant.py) with path_flags 0
 dev = torch.device("cuda", 0)
 n = 10 * 60 * SR
 x = synth_device(torch, C_PER_GPU, n, 0, dev)

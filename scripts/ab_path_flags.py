@@ -1,6 +1,6 @@
 """A/B of path_flags variants on config 2 (device-resident): step time, per-kernel times, and bit-equality of the outputs.
 
-    python scripts/ab_path_flags.py 0 8        # default vs k1 with cp.async-staged sample rows
+    python scripts/ab_path_flags.py 0 16       # default (dual kernels) vs one unit per warp
 """
 import os
 import sys
@@ -11,7 +11,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bench import synth_device, SR, C_PER_GPU  # noqa: E402
 from noisereduce_b200.device import DeviceGate  # noqa: E402
 
-flags = [int(a) for a in sys.argv[1:]] or [0, 8]
+flags = [int(a) for a in sys.argv[1:]] or [0, 16]
 dev = torch.device("cuda", 0)
 n = 10 * 60 * SR
 x = synth_device(torch, C_PER_GPU, n, 0, dev)

@@ -35,35 +35,29 @@ def _assert_stationary(res, exact_bits=True):
 
 def test_stationary_chunked_two_channels(lib):
     y = synth_small(C=2, n=12000)
-    cfg = O.GateConfig(sr=SR, stationary=True, chunk_size=5000, padding=600)
-    res = P.check_stationary(lib, y, cfg, tap_unit=(1, 1))
-    _assert_stationary(res)
-    assert res["stats"]["units"] == 6 and res["mask0_on_frac"] > 0.05
-    # last chunk (shorter valid span) and first chunk (left zero padding)
-    _assert_stationary(P.check_stationary(lib, y, cfg, tap_unit=(2, 0)))
-    _assert_stationary(P.check_stationary(lib, y, cfg, tap_unit=(0, 1)))
+    for pad in (600, 601):                              # 601: every sample row starts off a 16-byte boundary
+        cfg = O.GateConfig(sr=SR, stationary=True, chunk_size=5000, padding=pad)
+        res = P.check_stationary(lib, y, cfg, tap_unit=(1, 1))
+        _assert_stationary(res)
+        assert res["stats"]["units"] == 6 and res["mask0_on_frac"] > 0.05
+        # last chunk (shorter valid span) and first chunk (left zero padding)
+        _assert_stationary(P.check_stationary(lib, y, cfg, tap_unit=(2, 0)))
+        _assert_stationary(P.check_stationary(lib, y, cfg, tap_unit=(0, 1)))
 
 
-SR48 = 48000      # n_grad_freq = 5, n_grad_time = 9: the geometry of configs 2 / 5 -> single-pass fused kernel
-
-
-def test_spectrum_cache_and_recompute_paths_agree(lib):
-    """Default: k1 / k1n store the packed spectra and k2 loads them (no second forward FFT); path_flags bit 1
-    re-transforms instead.  Both are checked against the oracle and against each other."""
+def test_spectrum_cache_paths(lib):
+    """k1 / k1n store the packed spectra and k2 loads them (no second forward FFT), checked against the oracle."""
     y = synth_small(C=2, n=12000)
     for stationary in (True, False):
         cfg = O.GateConfig(sr=SR, stationary=stationary, chunk_size=5000, padding=600, time_constant_s=0.2, prop_decrease=0.9)
         chk = P.check_stationary if stationary else P.check_nonstationary
         a = chk(lib, y, cfg, tap_unit=(1, 1))
-        b = chk(lib, y, cfg, tap_unit=(1, 1), path_flags=2)
-        for r in (a, b):
-            assert r["mask_err"] < P.MASK_TOL_NONSTAT and r["out_relinf"] < P.OUT_TOL_TIGHT * 5
+        assert a["mask_err"] < P.MASK_TOL_NONSTAT and a["out_relinf"] < P.OUT_TOL_TIGHT * 5
         if stationary:
-            assert a["mask0_mismatch"] == 0 and b["mask0_mismatch"] == 0
+            assert a["mask0_mismatch"] == 0
     # odd first frame of a run, single chunk, tiny padding: pair alignment of the cached spectra
     cfg = O.GateConfig(sr=SR, stationary=True, chunk_size=2500, padding=0)
     _assert_stationary(P.check_stationary(lib, y[:1, :7000], cfg, tap_unit=(2, 0)))
-    _assert_stationary(P.check_stationary(lib, y[:1, :7000], cfg, tap_unit=(2, 0), path_flags=2))
 
 
 def test_pipelined_host_path_one_chunk_per_slab(lib):
@@ -179,8 +173,8 @@ def test_nonstationary_n_fft_2048(lib):
 
 def test_float_mask_box_smoothing_and_2k_spectrum_cache(lib):
     """k_smooth_box (1 <= nf <= 12: two sliding box sums per row) against the oracle and against the tap-loop
-    streaming kernel (path_flags 128); k2c_synthesize_2k (spectra cached by k1n_magnitude_2k) against the
-    re-transforming k2_synthesize_2k (path_flags 2).  The last case has config 3's filter extents (nf 10, nt 4)."""
+    streaming kernel (path_flags 128); k2c_synthesize_2k (spectra cached by k1n_magnitude_2k) against the oracle.
+    The last case has config 3's filter extents (nf 10, nt 4)."""
     y = synth_small(C=2, n=20000)
     cases = [(1024, 40, 20), (1024, 70, 70), (1024, 170, 150), (1024, 330, 40), (1024, 390, 100),
              (2048, 16, 40), (2048, 100, 300), (2048, 160, 130)]
@@ -194,11 +188,8 @@ def test_float_mask_box_smoothing_and_2k_spectrum_cache(lib):
     cfg = O.GateConfig(sr=SR, stationary=False, n_fft=2048, chunk_size=7000, padding=600, freq_mask_smooth_hz=160,
                        time_mask_smooth_ms=130)
     for unit in [(0, 0), (2, 1)]:
-        a = P.check_nonstationary(lib, y, cfg, tap_unit=unit)
-        b = P.check_nonstationary(lib, y, cfg, tap_unit=unit, path_flags=2)
-        for r in (a, b):
-            assert r["spec_err"] < P.SPEC_TOL and r["mask_err"] < P.MASK_TOL_NONSTAT and r["out_relinf"] < P.OUT_TOL_TIGHT * 5
-        assert abs(a["out_relinf"] - b["out_relinf"]) < 1e-6
+        r = P.check_nonstationary(lib, y, cfg, tap_unit=unit)
+        assert r["spec_err"] < P.SPEC_TOL and r["mask_err"] < P.MASK_TOL_NONSTAT and r["out_relinf"] < P.OUT_TOL_TIGHT * 5
     # the follower with its forward sweep stored (path_flags 64) instead of regenerated, odd batch remainders (T = 17, 30)
     for n, cs in [(4000, 0), (7400, 0)]:
         cfg = O.GateConfig(sr=SR, stationary=False, chunk_size=cs or None, padding=300, time_constant_s=0.5)
@@ -500,20 +491,6 @@ def test_operator_attributes_of_the_reference(lib, monkeypatch):
     assert sg.noise_thresh.shape == sg.mean_freq_noise.shape == sg.std_freq_noise.shape == (513,)
     assert np.abs(sg.noise_thresh - info["thresh"]).max() < P.THRESH_TOL_DB
     assert np.abs(sg.mean_freq_noise - info["noise_mean"]).max() < P.THRESH_TOL_DB
-
-
-def test_k1_staged_sample_rows_variant(lib):
-    """path_flags bit 3 (experimental): k1 streams the next pair's float32 rows into shared memory; 16-byte copies
-    when the rows are aligned, word copies otherwise; chunk / recording edges fall back to the direct loads."""
-    y = synth_small(C=2, n=12000)
-    for pad in (600, 601):                              # 601: every row starts off a 16-byte boundary
-        cfg = O.GateConfig(sr=SR, stationary=True, chunk_size=5000, padding=pad)
-        for tap in ((1, 1), (2, 0), (0, 0)):
-            r = P.check_stationary(lib, y, cfg, tap_unit=tap, path_flags=8)
-            _assert_stationary(r)
-    yi = np.round(y * 20000).astype(np.int16)           # not float32: the flag is ignored
-    r = P.check_stationary(lib, yi, O.GateConfig(sr=SR, stationary=True, chunk_size=5000, padding=600), tap_unit=(1, 0), path_flags=8)
-    assert r["mask0_mismatch"] == 0 and r["out_max_lsb"] <= 1
 
 
 def test_c_abi_argument_and_state_errors(lib):

@@ -59,9 +59,9 @@ def test_config2_shaped_chunks_mask_bit_exact(lib):
         _assert_stationary(res)
         assert res["T"] == 2579
         worst = max(worst, res["out_relinf"])
-    # the default path caches spectra between analysis and synthesis (dual kernels: two channels per warp); the
-    # re-transform variant (path_flags 2) and the one-unit-per-warp kernels (16) must agree with it and with the oracle
-    for flags in (2, 16):
+    # the default path runs the dual kernels (two channels per warp); the one-unit-per-warp kernels (path_flags 16)
+    # must agree with it and with the oracle
+    for flags in (16,):
         alt = P.check_stationary(lib, y, cfg, tap_unit=(1, 2), path_flags=flags)
         _assert_stationary(alt)
         assert P.relinf(res["out"], alt["out"]) < P.OUT_TOL_TIGHT
@@ -116,8 +116,8 @@ def test_nonstationary_n_fft_2048_config3(lib, golden_dir):
     out = nr.reduce_noise(y=s["y"].astype(np.float64), sr=int(s["sr"]), stationary=False, n_fft=2048,
                           time_constant_s=0.5, prop_decrease=0.9)
     assert out.dtype == np.float64 and P.relinf(out, s["out_nonstat_2048_f64"]) < P.OUT_TOL
-    # the kept variants: tap-loop smoothing (128), re-transforming synthesis (2), stored forward sweep (64)
-    for flags in (128, 2, 64):
+    # the forced paths: tap-loop smoothing (128), stored forward sweep (64)
+    for flags in (128, 64):
         res = P.check_nonstationary(lib, y, cfg, tap_unit=(1, 0), path_flags=flags)
         assert res["spec_err"] < P.SPEC_TOL and res["mask_err"] < P.MASK_TOL_NONSTAT, (flags, res)
         assert res["out_relinf"] < P.OUT_TOL_TIGHT * 5, (flags, res)
